@@ -73,7 +73,28 @@ def parse_args():
     ap.add_argument("--aggr", default="", help="run ONLY aggr(func(m[d])) by (label) as the main record, e.g. --aggr sum")
     ap.add_argument("--groups", type=int, default=1000, help="label groups for --aggr")
     ap.add_argument("--cpu-seconds", type=float, default=2.0, help="minimum wall time of the cpu_baseline measurement (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the result of the last one (rank 0) to DIR as float64 .npy files: "
+                         "result.npy (rows of the [series or groups x points] result, a fixed seeded sample when it exceeds "
+                         "%d MB), result_rows.npy (their row indices) and samples_scanned.npy" % (DUMP_BYTES // 1_000_000))
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_BYTES = 60_000_000  # result.npy stays below this; the three files of --dump-outputs stay below 64 MB
+
+
+def dump_outputs(dirname, rows_of, nrows, ncols, scanned):
+    """--dump-outputs: writes rows of a [nrows x ncols] result (rows_of(idx) -> float array) to DIR/result.npy.  The row
+    sample depends only on the shape, so two builds run with the same arguments write files that compare row for row."""
+    k = min(nrows, max(1, DUMP_BYTES // (8 * ncols)))
+    idx = np.arange(nrows) if k == nrows else np.sort(np.random.default_rng(0).choice(nrows, size=k, replace=False))
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "result.npy"), np.asarray(rows_of(idx), dtype=np.float64))
+    np.save(os.path.join(dirname, "result_rows.npy"), idx.astype(np.float64))
+    np.save(os.path.join(dirname, "samples_scanned.npy"), np.array([scanned], dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ oracle side (input + CPU arm)
@@ -373,6 +394,7 @@ class CpuArm:
                                         out.ctypes.data_as(self.O.f64p), C.byref(scanned), 1)
         dt = time.perf_counter() - t
         assert r == 0, r
+        self.scanned = scanned.value
         return dt
 
     def thread_candidates(self):
@@ -464,6 +486,8 @@ def main():
         descs, payload, _ = gen_blocks(a.blocks, a.rows, seed=1234, kind=a.kind, ts_kind=a.ts, encoder=a.encoder)
         arm = CpuArm(descs, payload, a.func, start, end, step, a.window_ms)
         m = arm.measure(steps=a.steps, warmup=a.warmup)  # per thread count: `warmup` untimed passes, then `steps` timed ones
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, lambda idx: arm.out[idx], a.blocks, arm.P, arm.scanned)
         out = dict(base)
         out.update({"impl": "reference", "value": m["value"], "ms_per_step": m["ms_per_pass"],
                     "cpu_baseline": m, "gpu_launches": 0,
@@ -601,6 +625,11 @@ def main():
     dev_ms_step, launches, (tb, te), last = time_steps(main_step, a.warmup, a.steps)
     scanned = last[1]
     clocks = sampler.window(tb, te)
+    if a.dump_outputs and rank == 0:  # before any later call reuses out_dev / the aggregate's host buffer
+        if a.aggr:
+            dump_outputs(a.dump_outputs, lambda idx: aggr_host[idx], a.groups, points, scanned)
+        else:
+            dump_outputs(a.dump_outputs, lambda idx: out_dev[torch.from_numpy(idx).cuda()].cpu().numpy(), a.blocks, points, scanned)
     # per-stage device times of one extra step (CUDA events inside the library, same stream)
     ctx.enable_stage_timing(True)
     main_step()
